@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Llama-2-7B int4 g128 greedy decode, batch 1 (BASELINE.json configs[1]); one step = one generated token.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 ours:       synthetic GPTQ-style weights (random nibbles, seed 1234, SURVEY.md section 8d), every op a kernel of
             libqbits_b200.so; one decode step = ONE launch of the persistent kernel k_decode_mega (csrc/mega.cu).
@@ -13,6 +13,13 @@ ours:       synthetic GPTQ-style weights (random nibbles, seed 1234, SURVEY.md s
             cpu_baseline = the oracle's C port of the reference CPU path on the box's host cores, bounded sample
 reference:  the same C port (oracle/woq_cpu.c: the reference's own kernels cannot be built offline) on all host threads.
 N > 1:      replicas only in this round (one engine per rank, no collective); value = sum over ranks.
+--dump-outputs DIR (ours, rank 0): after the timed steps, what each timed path handed back in its last step, as
+            DIR/<name>.npy (float32 / float64).  Weights, prompt and first token are seeded, so two builds run with the
+            same arguments can be compared output for output:
+            decode_resident_logits [1, vocab]  logits of the last device-resident step
+            decode_host_logits     [1, vocab]  logits of the last host-buffer step
+            decode_host_token      [1]         the token id that step returned
+            prefill_logits         [8, vocab]  last-position logits of the end-to-end prefill (absent without prefill)
 """
 import argparse
 import json
@@ -219,6 +226,16 @@ def run_reference(args, rank, world):
     }))
 
 
+def write_outputs(out_dir, outputs):
+    """Each tensor as out_dir/<name>.npy: float64 stays float64, every other dtype is stored as float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t if t.dtype == torch.float64 else t.float()).numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -257,6 +274,9 @@ def run_ours(args, rank, world, local_rank):
         ms_dev = eng.decode_resident(1, pos, args.steps)
         pos += args.steps
         barrier()
+        outputs = {}
+        if args.dump_outputs:
+            outputs["decode_resident_logits"] = eng.last_logits(1)
         # ---- end to end: host token in, host token out, every step
         tok = eng.decode_host(tok, pos)
         pos += 1
@@ -268,6 +288,9 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
         ms_e2e = (time.perf_counter() - t0) * 1e3
         barrier()
+        if args.dump_outputs:
+            outputs["decode_host_logits"] = eng.last_logits(1)
+            outputs["decode_host_token"] = torch.tensor(tok, dtype=torch.float64)
         # ---- dominant kernel family alone
         ms_lin, bytes_lin, n_lin = eng.time_linears(1, reps=5)
         # ---- prefill, B=8 x S=2048 (configs[2]): device time per op class by CUDA events, then end to end from host ids
@@ -292,6 +315,8 @@ def run_ours(args, rank, world, local_rank):
             first = torch.argmax(lg, dim=-1).cpu()                              # d2h of the first generated ids
             pre_e2e_ms = (time.perf_counter() - t0) * 1e3
             pre = (best, pre_e2e_ms, int(first[0]))
+            if args.dump_outputs:
+                outputs["prefill_logits"] = lg
             pre_clock = clk.window(t_pre0, time.perf_counter())
     launches = lib.qb_launch_count() - launches0
     # ---- N > 1 only: ONE model sharded over the N GPUs (Megatron column/row split, partial sums exchanged through NVLink peer
@@ -321,6 +346,8 @@ def run_ours(args, rank, world, local_rank):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -398,7 +425,12 @@ def main():
     ap.add_argument("--steps", type=int, default=128)
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed steps to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -121,13 +121,29 @@ def test_c_port_matches_numpy_oracle():
     assert cpu_port.threads() >= 1
 
 
-def test_bench_accounting_matches_survey():
+def _load_bench():
     import importlib.util
     spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
     b = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(b)
+    return b
+
+
+def test_bench_accounting_matches_survey():
+    b = _load_bench()
     assert b.algorithmic_bytes_per_token(0) == 3_238_002_688 + 101_187_584 + 262_144_000   # SURVEY.md section 8d
     assert b.algorithmic_bytes_per_token(10) - b.algorithmic_bytes_per_token(0) == 524_288 * 10
+
+
+def test_bench_dump_outputs_are_float32_or_float64(tmp_path):
+    b = _load_bench()
+    logits = torch.randn(2, 5).to(torch.bfloat16)
+    b.write_outputs(str(tmp_path / "out"), {"logits": logits, "token": torch.tensor([31999], dtype=torch.float64)})
+    assert sorted(os.listdir(tmp_path / "out")) == ["logits.npy", "token.npy"]
+    got = np.load(tmp_path / "out" / "logits.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, logits.float().numpy())
+    tok = np.load(tmp_path / "out" / "token.npy")
+    assert tok.dtype == np.float64 and tok.tolist() == [31999.0]
 
 
 def test_interleave_gate_up_layout():
