@@ -16,11 +16,15 @@ def _mk_lin(rng, K, N, group, asym):
     return dict(q=q, scale=s, zp=z)
 
 
-def _ref_forward(geom, layers, embed, fnorm, lm_head, tokens, group, stype, f64=False):
+def _ref_forward(geom, layers, embed, fnorm, lm_head, tokens, group, stype, f64=False, last=None, wround=0):
     """tokens [B, T] -> logits [B, T, V] in numpy with bf16 rounding at the points where the reference's bf16 modules round
     (module outputs, residual adds, RMSNorm, RoPE, attention output, SiLU, the gate * up product).  Matrix products
     accumulate in fp32 (BLAS) or, with f64=True, in fp64: the difference between the two is the test's own noise floor
-    (a bf16 rounding that flips on one side moves a logit by ~2^-9 of an activation; tools/parity_report.py records it)."""
+    (a bf16 rounding that flips on one side moves a logit by ~2^-9 of an activation; tools/parity_report.py records it).
+    last=n: logits [B, n, V] of the last n positions only; the last layer's attention queries, MLP and the lm_head then run
+    on those n rows (earlier layers still need every position for the keys and values).
+    wround=n: positions 0..n-1 multiply by the dequantised weights rounded to bf16, as the tensor-core GEMM that runs a
+    prefill of 64 rows or more does (gemm_tc.cu); later positions (decode steps: exact integer math, fp32 scaling) do not."""
     r = O.bf16_round
     if f64:
         class _M:  # matmul in fp64, result back in fp32
@@ -35,19 +39,29 @@ def _ref_forward(geom, layers, embed, fnorm, lm_head, tokens, group, stype, f64=
     cos, sin = O.rope_cos_sin(np.arange(T), D, geom.rope_theta)
     cos, sin = r(cos), r(sin)
     deq = lambda l: O.dequantize(l["q"], l["scale"], l["zp"], group, "int4_clip", stype)
-    for L in layers:
+
+    def mm(x, l):   # x [B, rows, K]: the last `rows` positions
+        w = deq(l)
+        n = min(max(wround - (T - x.shape[1]), 0), x.shape[1])
+        if n == 0:
+            return wrap(x) @ w
+        return np.concatenate([wrap(x[:, :n]) @ r(w), wrap(x[:, n:]) @ w], axis=1)
+
+    for li, L in enumerate(layers):
         x = r(r(O.rmsnorm(h, np.ones_like(L["an"]), geom.rms_eps)) * L["an"])
-        q = r(wrap(x) @ deq(L["q"])).reshape(B, T, Hq, D).transpose(0, 2, 1, 3)
-        k = r(wrap(x) @ deq(L["k"])).reshape(B, T, Hkv, D).transpose(0, 2, 1, 3)
-        v = r(wrap(x) @ deq(L["v"])).reshape(B, T, Hkv, D).transpose(0, 2, 1, 3)
+        q = r(mm(x, L["q"])).reshape(B, T, Hq, D).transpose(0, 2, 1, 3)
+        k = r(mm(x, L["k"])).reshape(B, T, Hkv, D).transpose(0, 2, 1, 3)
+        v = r(mm(x, L["v"])).reshape(B, T, Hkv, D).transpose(0, 2, 1, 3)
         rope = lambda t: r(r(t * cos[None, None]) + r(O.rotate_half(t) * sin[None, None]))
         q, k = rope(q), rope(k)
-        a = r(O.attention(q, k, v, causal=True)).transpose(0, 2, 1, 3).reshape(B, T, Hq * D)
-        h = r(h + r(wrap(a) @ deq(L["o"])))          # the module output is bf16 before `residual + hidden` (HF LlamaDecoderLayer)
+        if last is not None and li == len(layers) - 1:   # queries at positions T - last .. T - 1 (O.attention's default offset)
+            q, h = q[:, :, T - last:], h[:, T - last:]
+        a = r(O.attention(q, k, v, causal=True)).transpose(0, 2, 1, 3).reshape(B, q.shape[2], Hq * D)
+        h = r(h + r(mm(a, L["o"])))          # the module output is bf16 before `residual + hidden` (HF LlamaDecoderLayer)
         x = r(r(O.rmsnorm(h, np.ones_like(L["mn"]), geom.rms_eps)) * L["mn"])
-        g, u = r(wrap(x) @ deq(L["gate"])), r(wrap(x) @ deq(L["up"]))
+        g, u = r(mm(x, L["gate"])), r(mm(x, L["up"]))
         m = r(r(O.silu(g)) * u)                 # act_fn(gate_proj(x)) * up_proj(x): every op rounds to bf16 (HF LlamaMLP)
-        h = r(h + r(wrap(m) @ deq(L["down"])))
+        h = r(h + r(mm(m, L["down"])))
     x = r(r(O.rmsnorm(h, np.ones_like(fnorm), geom.rms_eps)) * fnorm)
     return wrap(x) @ lm_head.T
 
